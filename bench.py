@@ -19,6 +19,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 WORKLOADS = {
     # name: (env, algo, lanes/GPU, horizon, hidden, alg bytes per env step (SURVEY 8d: 4*(O+3A+1)+1))
@@ -141,6 +142,42 @@ def cpu_arm(workload, steps, warmup, cores=None, sample_steps=None, seconds_budg
     return value, info, sum(times) / len(times) * 1e3
 
 
+def dump_outputs(out_dir, algo, policy, baseline, lanes_budget_bytes=32 << 20):
+    """--dump-outputs: what the last timed iteration hands back to its caller, one .npy file per array in out_dir.
+      policy_params, baseline_coeffs  float64, after that iteration's update and baseline fit
+      stat_<key>                      float64 scalars, the iteration's logger.record_tabular table
+      observations, actions, means    float32, [dim][T][lane] as the device holds them, for a fixed, seeded sample of
+      rewards, advantages, returns,   this rank's lanes (at most lanes_budget_bytes in all); flags are the FLAG_* bits
+      baselines, flags                of include/b200rl.h, masked samples included
+      lanes                           float64, global index of each sampled lane
+    The inputs of the iteration follow from the arguments and fixed seeds alone, so two builds run with the same
+    arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    from rllab_b200.misc import logger
+    b = algo.sampler.batch
+    out = dict(policy_params=np.asarray(policy.get_param_values(), dtype=np.float64))
+    coeffs = baseline.get_param_values()
+    if coeffs is not None:
+        out["baseline_coeffs"] = np.asarray(coeffs, dtype=np.float64)
+    for k, v in logger.get_last_table().items():
+        if isinstance(v, (int, float, np.number)):
+            out["stat_" + k] = np.float64(v)
+    planes = dict(observations=b.obs, actions=b.act, means=b.mean, rewards=b.rew, advantages=b.adv, returns=b.ret,
+                  baselines=b.base, flags=b.flags)
+    per_lane = 4 * b.T * sum(t.numel() // (b.T * b.N) for t in planes.values())
+    n_sample = min(b.N, max(1, lanes_budget_bytes // per_lane))
+    idx = np.sort(np.random.RandomState(0).choice(b.N, n_sample, replace=False))
+    sel = torch.as_tensor(idx, device=b.device)
+    for name, t in planes.items():
+        out[name] = t.index_select(t.dim() - 1, sel).cpu().numpy().astype(np.float32)
+    out["lanes"] = (idx + algo.sampler.lane0).astype(np.float64)
+    assert sum(a.nbytes for a in out.values()) <= 64 << 20
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -153,6 +190,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the short TRPO workloads reported under extra.workloads")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed iteration computed to DIR/<name>.npy (see dump_outputs)")
     ap.add_argument("--cpu-arm-json", action="store_true", help=argparse.SUPPRESS)   # internal: CPU leg in a clean process
     args = ap.parse_args()
     assert args.warmup >= 0 and args.steps >= 1
@@ -256,6 +295,8 @@ def main():
     collectives = (comm.n_collectives - c0) / args.steps            # NCCL collectives on the iteration's critical path
     peer_exchanges = (comm.n_peer_exchanges - x0) / args.steps      # peer-memory exchanges (fused or stand-alone kernels)
     itr += args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, algo, policy, baseline)
     d2h0 = ops.PendingHost.bytes_total
     ms_e2e = run(algo, policy, args.steps, itr, True)
     d2h_stats = (ops.PendingHost.bytes_total - d2h0) / args.steps    # statistics / loss triples read back per iteration
