@@ -150,3 +150,47 @@ def test_rollout_is_deterministic_and_shard_invariant(full):
     other = ops.LaneBatch(4, 1, n, 64, dev)
     ops.rollout(L.ENV_CARTPOLE, th32, H, H, 1e-6, other, 64, None, None, 5, 10, 0)      # next iteration: new noise
     assert not torch.equal(ref.act, other.act)
+
+
+def test_gradient_and_fisher_product_match_f64_kernels(full):
+    """float32 TRPO gradient and cached Fisher product at cfg2 size against update_f64 (pinned to the float64 oracle by
+    tests/test_gpu_multitile.py), in relative norm: ~26 000 tiles per pass, every CTA loops hundreds of times.  Measured
+    on one B200: see DESIGN.md §5."""
+    from test_gpu_multitile import TOL, _f32_vs_f64
+    L, ops, b, th32 = full["L"], full["ops"], full["b"], full["th32"]
+    x = np.random.RandomState(4).randn(full["dims"].P).astype(np.float32).astype(np.float64)
+    err_g, err_H = _f32_vs_f64(ops, L, b, (4, H, H, 1), th32, x)
+    print("\ncfg2: grad err %.3e  fvp err %.3e" % (err_g, err_H))
+    assert err_g <= TOL["grad"] and err_H <= TOL["fvp"], (err_g, err_H)
+
+
+def test_lfb_gram_and_fit_match_host_float64(full):
+    """LinearFeatureBaseline normal equations over all 13.1 M samples against a float64 Gram accumulated on the host in
+    chunks, and the device solve's predictions against the host's lstsq on that Gram."""
+    from oracle import sampler as S
+    ops, b, dev = full["ops"], full["b"], full["dev"]
+    d1 = 2 * 4 + 5
+    gram = torch.empty((d1 * (d1 + 1) // 2,), dtype=torch.float64, device=dev)
+    ops.lfb_gram(b, gram)
+    obs = b.obs.cpu().numpy().reshape(4, -1)
+    ts = b.tstep.cpu().view(torch.int16).numpy().view(np.uint16).reshape(-1)
+    ret = b.ret.cpu().numpy().reshape(-1)
+    G = np.zeros((d1, d1))
+    step = 1 << 20
+    for i in range(0, N * T, step):
+        F = np.concatenate([S.lfb_features_lanes(obs[:, i:i + step, None], ts[i:i + step, None])[:, :, 0],
+                            ret[None, i:i + step].astype(np.float64)], axis=0)
+        G += F @ F.T
+    iu = np.triu_indices(d1)
+    np.testing.assert_allclose(gram.cpu().numpy(), G[iu], rtol=2e-6, atol=1e-6 * np.abs(G).max())
+    w_dev = torch.empty((d1 - 1,), dtype=torch.float64, device=dev)
+    info = torch.zeros((3,), dtype=torch.float64, device=dev)
+    ops.lfb_solve(4, gram, 1e-5, w_dev, info)
+    reg, _, ok = info.cpu().tolist()
+    assert ok == 1.0
+    w_ref = S.lfb_fit_normal(G[:-1, :-1], G[:-1, -1], reg)
+    sel = np.random.RandomState(0).choice(N * T, 1 << 20, replace=False)
+    Fs = S.lfb_features_lanes(obs[:, sel, None], ts[sel, None])[:, :, 0].T
+    pred, pred_ref = Fs @ w_dev.cpu().numpy(), Fs @ w_ref
+    # Cholesky (device) and lstsq (host) on the same ill-conditioned d = 12 system: agree to 1e-3 of the prediction range
+    assert np.abs(pred - pred_ref).max() <= 1e-3 * np.abs(pred_ref).max()

@@ -137,7 +137,7 @@ def test_env_step_matches_oracle(dev, env_name):
 
 
 # ------------------------------------------------------------------------------------------- fused rollout
-@pytest.mark.parametrize("env_name,hidden", [(e, 32) for e in ENVS] + [("cartpole", 64)])
+@pytest.mark.parametrize("env_name,hidden", [(e, 32) for e in ENVS] + [(e, 64) for e in ENVS])
 def test_rollout_matches_oracle(dev, env_name, hidden):
     N, T, mpl = 256, 40, 17
     env, dims, theta, b, eps, rr = _gpu_rollout(env_name, hidden, N, T, mpl, dev)
@@ -292,15 +292,25 @@ def test_process_samples_matches_reference_golden(dev, golden):
         np.testing.assert_allclose(pred_solve, pred_ref, rtol=2e-3, atol=2e-3)
 
 
-@pytest.mark.parametrize("env_name", ["cartpole", "pendulum"])
-def test_process_samples_matches_oracle_large(dev, env_name):
+@pytest.mark.parametrize("drop_cut", [False, True], ids=["keep-cut", "drop-cut"])
+@pytest.mark.parametrize("N,T", [(4099, 101), (4096, 128)], ids=["unaligned", "aligned"])
+@pytest.mark.parametrize("env_name", ENVS)
+def test_process_samples_matches_oracle_large(dev, env_name, N, T, drop_cut):
+    """The baseline chain at every compiled obs_dim (2, 3, 4, 6, 13, 20) with a nonzero baseline w: predictor, GAE scan,
+    statistics, centring, Gram and the device solve (d = 2O+4 up to 44).  4099 x 101: B % 4 != 0 (scalar predictor,
+    unaligned scan); 4096 x 128: the vector predictor and the staged scan.  Both sizes make every Gram kernel's
+    grid-stride loop iterate."""
     ops = _ops()
-    N, T, mpl = 1024, 64, 40
+    mpl = 40
     env, dims, theta, b, eps, rr = _gpu_rollout(env_name, 32, N, T, mpl, dev)
     traj = b.to_numpy()
     w = np.random.RandomState(5).randn(2 * env.O + 4) * 0.3
-    ops.process_samples(b, torch.tensor(w, dtype=torch.float64, device=dev), 0.99, 0.95)
-    ref = S.process_samples_lanes(traj, w, 0.99, 0.95, center_adv=True)
+    ops.process_samples(b, torch.tensor(w, dtype=torch.float64, device=dev), 0.99, 0.95, drop_cut_paths=drop_cut)
+    ref = S.process_samples_lanes(traj, w, 0.99, 0.95, center_adv=True, drop_cut=drop_cut)
+    valid = ref["valid"]
+    if drop_cut:
+        assert not valid.all()
+        assert np.array_equal((b.flags.cpu().numpy() & S.FLAG_MASKED) != 0, ~valid)
     np.testing.assert_allclose(b.ret.cpu().numpy(), ref["ret"], rtol=1e-5, atol=1e-4)
     np.testing.assert_allclose(b.base.cpu().numpy(), ref["base"], rtol=1e-5, atol=1e-4)
     np.testing.assert_allclose(b.adv.cpu().numpy(), ref["adv_raw"], rtol=1e-5, atol=2e-4)
@@ -309,26 +319,29 @@ def test_process_samples_matches_oracle_large(dev, env_name):
                 "adv_mean", "adv_std"):
         np.testing.assert_allclose(st[key], ref["stats"][key], rtol=1e-6, atol=1e-6, err_msg=key)
     assert st["NumTrajs"] == ref["stats"]["NumTrajs"]
+    assert b.sums.cpu().numpy()[2] == valid.sum()
     ops.center_advantages(b, True, False)
     np.testing.assert_allclose(b.adv.cpu().numpy(), ref["adv"], rtol=1e-4, atol=1e-5)
     d1 = 2 * b.O + 5
     gram = torch.empty((d1 * (d1 + 1) // 2,), dtype=torch.float64, device=dev)
     ops.lfb_gram(b, gram)
+    keep = valid.reshape(-1)
     F = S.lfb_features_lanes(traj["obs"], traj["tstep"]).reshape(d1 - 1, -1)
-    F = np.concatenate([F, ref["ret"].reshape(1, -1)], axis=0)
+    F = np.concatenate([F, ref["ret"].reshape(1, -1)], axis=0)[:, keep]
     G = (F @ F.T)[np.triu_indices(d1)]
     np.testing.assert_allclose(gram.cpu().numpy(), G, rtol=2e-5, atol=1e-3)
     # device solve == the reference's lstsq on the same regularised normal equations
     w_dev = torch.empty((d1 - 1,), dtype=torch.float64, device=dev)
     info = torch.zeros((3,), dtype=torch.float64, device=dev)
     ops.lfb_solve(b.O, gram, 1e-5, w_dev, info)
+    reg, _, ok = info.cpu().tolist()
+    assert ok == 1.0
     Gf = np.zeros((d1, d1))
     Gf[np.triu_indices(d1)] = gram.cpu().numpy()
     Gf = Gf + Gf.T - np.diag(np.diag(Gf))
-    w_ref = S.lfb_fit_normal(Gf[:-1, :-1], Gf[:-1, -1])
+    w_ref = S.lfb_fit_normal(Gf[:-1, :-1], Gf[:-1, -1], reg)
     Fm = F[:-1].T
     np.testing.assert_allclose(Fm @ w_dev.cpu().numpy(), Fm @ w_ref, rtol=1e-6, atol=1e-6)
-    assert info.cpu().tolist()[1:] == [0.0, 1.0]
 
 
 def test_lfb_solve_regularisation_retry(dev):
@@ -537,13 +550,14 @@ def test_f64_parity_kernels_match_oracle(dev, env_name, hidden):
     np.testing.assert_allclose(Hx.cpu().numpy(), ref_Hx, rtol=1e-8, atol=1e-12 * np.abs(ref_Hx).max())
 
 
-@pytest.mark.parametrize("O,A", [(6, 1), (13, 2), (20, 3), (4, 1)])
+@pytest.mark.parametrize("O,A", [(6, 1), (13, 2), (20, 3), (4, 1), (3, 1), (2, 2)])
 def test_lfb_gram_matches_numpy_on_synthetic_batches(dev, O, A):
     """LinearFeatureBaseline normal equations (linear_feature_baseline.py:19-37) on a synthetic batch for every compiled
     obs_dim: the register-tiled kernel (obs_dim 6 / 13 / 20), the register-triangle kernel (<= 4), ragged sizes (B not a
-    multiple of the 128-sample tile or of 4), masked samples, observations beyond the +-10 clip."""
+    multiple of the 128-sample tile or of 4), masked samples, observations beyond the +-10 clip; 4099 x 101 and
+    4096 x 128 make the grid-stride loops iterate (the float32 register triangle accumulates over the whole loop)."""
     ops, L = _ops(), _L()
-    for N, T in ((200, 37), (128, 64), (333, 5)):
+    for N, T in ((200, 37), (128, 64), (333, 5), (4099, 101), (4096, 128)):
         rng = np.random.RandomState(O * 100 + N)
         b = ops.LaneBatch(O, A, N, T, dev)
         obs = (rng.randn(O, T, N) * 6.0).astype(np.float32)
